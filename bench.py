@@ -61,7 +61,13 @@ def parse_args():
     ap.add_argument("--no-points", action="store_true", help="skip the 16384 / 65536-env points of the env-step roofline")
     ap.add_argument("--workload", default="smpl", choices=sorted(WORKLOADS), help="configuration of the headline numbers (default: the one the metric is quoted on)")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary configurations (H1, PNN big nets) reported as extra_configs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed epochs, write what the last one computed to DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "phc_b200":
+        ap.error("--dump-outputs needs --impl phc_b200")
+    return args
 
 
 def measured_peak_gbs():
@@ -319,7 +325,7 @@ def timed_epochs(agent, steps: int, warmup: int, world: int, read_result: bool):
     l0 = lib.phc_launch_count()
     ev0.record()
     for _ in range(steps):
-        agent.train_epoch()
+        out = agent.train_epoch()
         if read_result:
             agent.train_result_dict()            # device->host read of the epoch's last losses (e2e mode)
     ev1.record()
@@ -332,7 +338,37 @@ def timed_epochs(agent, steps: int, warmup: int, world: int, read_result: bool):
         t = torch.tensor([ms], device=agent.device)
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
         ms = float(t.item())
-    return ms / steps, launches
+    return ms / steps, launches, out
+
+
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(agent, epoch_out, out_dir: str) -> None:
+    """--dump-outputs: what the last timed epoch returned (train_epoch's tensors, the last minibatch's losses) and what it left to
+    its caller (network parameters, normaliser statistics), one float32 / float64 array per file.  The inputs are seeded, so two
+    builds run with the same arguments can be compared file by file.  Between two runs of the same build the environment outputs
+    are bit-identical; the learner's atomically accumulated reductions differ in the last bits, which 3 + 5 epochs of training
+    grow to ~1e-4 relative in losses and weights (B200, 1000 W power limit).  The files share DUMP_BYTES smallest first; an array
+    larger than its share is replaced by a fixed sample of its flattened elements (the same seeded indices in every run)."""
+    import numpy as np
+    arrays = {f"epoch.{k}": v for k, v in epoch_out.items() if torch.is_tensor(v)}
+    arrays.update({f"loss.{k}": torch.tensor(v, dtype=torch.float64) for k, v in agent.train_result_dict().items()})
+    arrays.update({f"model.{k}": v for k, v in agent.model.state_dict().items()})
+    for name, sd in agent.get_stats_weights().items():
+        arrays.update({f"stats.{name}.{k}": v for k, v in sd.items()})
+    arrays = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32) for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    budget, left = DUMP_BYTES, len(arrays)
+    for name in sorted(arrays, key=lambda k: arrays[k].numel() * arrays[k].element_size()):
+        t = arrays[name]
+        keep = (budget // left - 128) // t.element_size()          # 128 bytes: the .npy header
+        if t.numel() > keep:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t.reshape(-1)[idx]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, t.numpy())
+        budget, left = budget - os.path.getsize(path), left - 1
 
 
 def env_kernel_roofline(task, peak_gbs: float, peak_src: str, iters: int = 40, algo_bytes: int = ALGO_BYTES_PER_ENV_STEP,
@@ -495,7 +531,7 @@ def run_extra_config(name: str, device, rank: int, world: int, peak_gbs: float, 
     w = WORKLOADS[name]
     try:
         agent, task = build_agent(w["envs"], device, rank, world, host_bank=False, workload=name)
-        ms, launches = timed_epochs(agent, steps, warmup, world, read_result=False)
+        ms, launches, _ = timed_epochs(agent, steps, warmup, world, read_result=False)
         out = {"workload": f"PPO epoch: {w['envs']} envs/GPU x 32 steps, {w['desc']}, minibatch 16384 x 6 mini-epochs", "num_envs_per_gpu": w["envs"],
                "value": HORIZON * w["envs"] * world / (ms * 1e-3), "unit": "env-steps/s", "ms_per_step": ms, "steps": steps, "warmup": warmup,
                "gpu_launches": int(launches), "dtype": "tf32 single pass (MLPs), f32 elsewhere" if name.endswith("_tf32") else "f32"}
@@ -528,12 +564,14 @@ def main():
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         torch.distributed.init_process_group("nccl", device_id=device)
-    import __graft_entry__
-    if rank == 0:
-        __graft_entry__.build()
-    if world > 1:
-        torch.distributed.barrier()
+    # the library __graft_entry__.build() left in the tree; the bench itself compiles nothing (the tree may be read-only)
+    from phc_b200 import _lib
+    if _lib.load().phc_compiled_sm() != 100:
+        raise SystemExit(f"bench.py: {_lib.LIB_PATH} was not compiled for sm_100a")
 
+    # the synthetic data is seeded; this seeds what the run draws from torch's global generators (reset times, action noise,
+    # minibatch order), so the same arguments give the same inputs in every run
+    torch.manual_seed(rank)
     sampler = ClockSampler(local)
     note("building agent (device-resident simulator snapshots)")
     wl = WORKLOADS[args.workload]
@@ -543,9 +581,12 @@ def main():
     note("agent built; timed epochs")
     if rank == 0:
         sampler.start()
-    sec_per_step, launches = timed_epochs(agent, args.steps, args.warmup, world, read_result=False)
+    sec_per_step, launches, last_epoch = timed_epochs(agent, args.steps, args.warmup, world, read_result=False)
     clocks = sampler.stop() if rank == 0 else None
     note(f"value arm done: {sec_per_step:.1f} ms/epoch")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(agent, last_epoch, args.dump_outputs)
+        note(f"outputs of the last timed epoch written to {args.dump_outputs}")
     if os.environ.get("PHC_PHASE_TIMING", "0") == "1" and rank == 0:       # diagnostic only: CUDA-event phase breakdown of one epoch
         agent.timer.report()
         agent.train_epoch()
@@ -572,7 +613,7 @@ def main():
     if not args.no_e2e:
         agent2, task2 = build_agent(args.num_envs, device, rank, world, host_bank=True, workload=args.workload)
         note("e2e agent built (pinned host snapshots)")
-        ms2, _ = timed_epochs(agent2, max(1, args.steps), max(3, args.warmup) if args.warmup >= 3 else args.warmup, world, read_result=True)
+        ms2, _, _ = timed_epochs(agent2, max(1, args.steps), max(3, args.warmup) if args.warmup >= 3 else args.warmup, world, read_result=True)
         e2e = {"value": env_steps / (ms2 * 1e-3), "unit": "env-steps/s", "ms_per_step": ms2,
                "h2d_bytes_per_step": HORIZON * task2.sim.h2d_bytes_per_step, "d2h_bytes_per_step": 16 * 4,
                "note": "simulator state (rigid bodies, dof state, dof forces) copied from pinned host memory every env step; epoch losses read back"}

@@ -26,6 +26,8 @@ What is executed on the reference side (no restatement involved):
   fut.npz      fut_tracks with 3 future samples (the [B, T, J*24] layout of compute_imitation_observations_v6)
   reset.npz    HumanoidAMP._init_amp_obs_ref, MotionLibBase.sample_time_interval
   g1.npz, smplx.npz   the h1.npz / envstep.npz recipes at the shipped shapes beyond 32 bodies (Unitree G1 38 + 1, SMPL-X 52)
+  replay.npz   ReplayBuffer.store / sample (phc/learning/replay_buffer.py)
+  dropin_signatures.json   positional parameters of the HumanoidIm / AMPAgent methods the drop-in mirrors line up with
 
   python tests/golden/make_golden.py load getup      # regenerate selected files only
 """
@@ -441,12 +443,22 @@ def gen_mcp():
     env._physics_step = lambda: None
     env.post_physics_step = lambda: None
     env.dr_randomizations = {}
+    # the primitives' outputs inside step are recorded too: the mixing is pinned bit for bit on them, independent of the
+    # host's CPU matmul rounding
+    pnn_forward = env.pnn.forward
+
+    def recording_forward(x, idx=-1):
+        out = pnn_forward(x, idx)
+        got["prim"] = torch.stack(out[1], dim=0)
+        return out
+    env.pnn.forward = recording_forward
     weights = torch.relu(torch.randn(N, K))                # composer output ends in a ReLU
     d["rms_mean"], d["rms_var"], d["obs_buf"], d["weights"] = rms["running_mean"], rms["running_var"], env.obs_buf, weights
     for disc in (False, True):
         env.discrete_mcp = disc
         env.step(weights)
         d["actions_discrete" if disc else "actions"] = got["actions"]
+        d["step_prim"] = got["prim"]
 
     # composer (amp_network_mcp_builder.py:57-63) rebuilt by the reference's own loader: ReLU after the last Linear
     comp = {"a2c_network.composer.0.weight": torch.randn(units[0], obs_dim) * 0.2, "a2c_network.composer.0.bias": torch.randn(units[0]) * 0.1,
@@ -738,6 +750,49 @@ def gen_load():
     save("load.npz", d)
 
 
+# ------------------------------------------------------------------------------------------------
+def gen_replay():
+    """ReplayBuffer (phc/learning/replay_buffer.py): circular store, the pre-fill `% head` rule, the permutation refresh.  The
+    buffer draws its permutations from the global generator seeded with 5; the stored rows come from their own generator."""
+    from phc.learning.replay_buffer import ReplayBuffer
+    from tests.test_replay_buffer_cpu import SAMPLE_SIZES, STORE_SIZES
+    size, width = 50, 7
+    torch.manual_seed(5)
+    ref = ReplayBuffer(size, "cpu")
+    g = torch.Generator().manual_seed(1)
+    d = dict(size=np.int64(size))
+    for step, n in enumerate(STORE_SIZES):
+        rows = torch.randn(n, width, generator=g)
+        ref.store({"amp_obs": rows})
+        d[f"rows{step}"], d[f"total{step}"], d[f"data{step}"] = rows, np.int64(ref.get_total_count()), ref._data_buf["amp_obs"].clone()
+        for k in SAMPLE_SIZES:
+            d[f"sample{step}_{k}"] = ref.sample(k)["amp_obs"]
+    save("replay.npz", d)
+
+
+def gen_dropin():
+    """Positional parameters (name, required) of the HumanoidIm / AMPAgent methods the mirrors must accept the same way."""
+    import importlib
+    import inspect
+    import json
+    from tests.test_dropin_surface import SIGNATURE_METHODS
+    classes = {"HumanoidIm": importlib.import_module("phc.env.tasks.humanoid_im").HumanoidIm,
+               "AMPAgent": importlib.import_module("phc.learning.amp_agent").AMPAgent}
+    out = {}
+    for cname, names in SIGNATURE_METHODS.items():
+        cls = classes[cname]
+        out[cname] = {}
+        for n in names:
+            assert any(n in vars(b) for b in cls.__mro__), f"reference lacks {cname}.{n}"
+            out[cname][n] = [[p.name, p.default is p.empty] for p in inspect.signature(getattr(cls, n)).parameters.values()
+                             if p.kind in (p.POSITIONAL_ONLY, p.POSITIONAL_OR_KEYWORD)]
+    path = os.path.join(HERE, "dropin_signatures.json")
+    with open(path, "w") as f:               # one line per method
+        f.write("{\n" + ",\n".join(f' "{c}": {{\n' + ",\n".join(f'  "{n}": {json.dumps(v)}' for n, v in m.items()) + "\n }"
+                                   for c, m in out.items()) + "\n}\n")
+    print(f"wrote {path}")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1:
         for name in sys.argv[1:]:
@@ -752,6 +807,8 @@ if __name__ == "__main__":
     gen_load()
     gen_getup()
     gen_fut()
+    gen_replay()
+    gen_dropin()
     gen_reset()
     gen_g1()
     gen_smplx()
